@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU)
   python bench.py --impl reference ...                      # the reference's CPU algorithm (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch: Vits.inference on a [32, 64] token batch per GPU
 (random-init VitsConfig, LJSpeech-shaped synthetic tokens), i.e. text encoder -> stochastic duration predictor
@@ -122,6 +123,27 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(self.NAMES) if any(len(r) > 2 + i and r[2 + i] == "Active" for r in self.rows)]
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm), "source": "nvml" if self.nvml else "nvidia-smi"}
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out, directory):
+    """Writes every tensor of one Vits.inference result as <directory>/<name>.npy, floating-point ones as float32 and
+    integer ones as float64 (exact), so two builds can be compared output for output.  Should they exceed DUMP_BYTES in
+    all, each array is cut to the same fixed, seeded sample of its flattened values in every run."""
+    import numpy as np
+    import torch
+    arrays = {k: v.detach().cpu().numpy().astype(np.float32 if v.is_floating_point() else np.float64)
+              for k, v in out.items() if torch.is_tensor(v)}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 1024 * len(arrays)           # room for the .npy headers
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        if total > budget:
+            n = max(1, a.size * budget // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        np.save(os.path.join(directory, k + ".npy"), a)
 
 
 def build_model(seed=1234):
@@ -470,6 +492,8 @@ def run_cuda(args):
         padded_samples += out["model_outputs"].numel()
         frames_padded += out["y_mask"].shape[0] * out["y_mask"].shape[-1]
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     samples_rank = int(sum(int(l.sum().item()) for l in lens_out))
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop(first_sample)
@@ -631,6 +655,8 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (float32 / float64 .npy files, at most 64 MB in all)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

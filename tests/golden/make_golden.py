@@ -15,6 +15,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+import fixtures  # noqa: E402
 import ref_import  # noqa: E402
 
 R = ref_import.load()
@@ -41,6 +42,7 @@ def save(name, obj):
 
 @torch.no_grad()
 def main():
+    torch.set_num_threads(fixtures.THREADS)
     torch.manual_seed(1234)
     H = R["hifigan"].HifiganGenerator
     # 1. HiFiGAN v1 topology, narrow channels, standalone vocoder flavour
@@ -253,6 +255,237 @@ def main_r02():
     save("tokenizer_cases", {"texts": texts, "graphemes": {"characters": g.characters, "punctuations": g.punctuations,
                                                            "pad": g.pad, "eos": g.eos, "bos": g.bos, "blank": g.blank},
                              "vocab": list(g.vocab), "cases": tok_cases})
+    main_full_width()
+    main_real_model()
+    main_reference_objects()
+
+
+def _regenerate(m, seed):
+    """Replaces the module's weights by the compact fixture's regenerated ones; returns what the fixture stores."""
+    # the discriminator of the Vits model is training-only: it keeps its own initialisation and stays out of the fixture
+    stats = fixtures.state_stats({k: v for k, v in m.state_dict().items() if not k.startswith("disc.")})
+    m.load_state_dict(fixtures.state_from_stats(stats, seed), strict=False)
+    return {"stats": stats, "seed": seed}
+
+
+@torch.no_grad()
+def main_full_width():
+    """The reference layer modules at full VITS width (tests/test_oracle_vs_reference.py): weights regenerated from
+    per-entry statistics of the reference's own initialisation, inputs re-drawn from fixed seeds by the test."""
+    cases = {}
+    torch.manual_seed(0)
+    m = R["hifigan"].HifiganGenerator(192, 1, "1", [[1, 3, 5]] * 3, [3, 7, 11], [16, 16, 4, 4], 512, [8, 8, 2, 2],
+                                      inference_padding=0, cond_channels=256, conv_pre_weight_norm=False,
+                                      conv_post_weight_norm=False, conv_post_bias=False).eval()
+    c = _regenerate(m, 1000)
+    torch.manual_seed(10)
+    x, g = torch.randn(1, 192, 6), torch.randn(1, 256, 1)
+    c["y"] = fixtures.record(m(x, g))
+    cases["hifigan"] = c
+
+    torch.manual_seed(1)
+    te = R["networks"].TextEncoder(100, 192, 192, 768, 2, 6, 3, 0.1).eval()
+    c = {"text_encoder": _regenerate(te, 2000)}
+    torch.manual_seed(11)
+    tok, lens = torch.randint(0, 100, (3, 21)), torch.tensor([21, 13, 5])
+    ref = te(tok, lens)
+    c["text_encoder_out"] = [fixtures.record(t) for t in ref]
+    sdp = R["sdp"].StochasticDurationPredictor(192, 192, 3, 0.5, 4, cond_channels=256).eval()
+    perturb_zero_params(sdp)
+    c["sdp"] = _regenerate(sdp, 3000)
+    torch.manual_seed(12)
+    g = torch.randn(3, 256, 1)
+    torch.manual_seed(9)           # the reference draws the SDP noise inside forward (sdp.py:287)
+    c["logw"] = fixtures.record(sdp(ref[0], ref[3], g=g, reverse=True, noise_scale=1.0))
+    fl = R["networks"].ResidualCouplingBlocks(192, 192, 5, 1, 4, cond_channels=256).eval()
+    perturb_zero_params(fl)
+    c["flow"] = _regenerate(fl, 4000)
+    torch.manual_seed(13)
+    z = torch.randn(3, 192, 40)
+    mask = seq_mask(torch.tensor([40, 22, 3]), 40)
+    c["flow_out"] = fixtures.record(fl(z, mask, g=g, reverse=True))
+    cases["vits_stack"] = c
+
+    rng = np.random.RandomState(0)
+    v = torch.from_numpy(rng.randn(8, 200, 1000).astype(np.float32))
+    t_x = torch.from_numpy(rng.randint(100, 201, size=8))
+    t_y = torch.tensor([int(rng.randint(5 * int(a) if 5 * int(a) <= 1000 else 1000, 1001)) for a in t_x])
+    mask = ((torch.arange(200)[None, :, None] < t_x[:, None, None]) &
+            (torch.arange(1000)[None, None, :] < t_y[:, None, None])).float()
+    assert R["helpers"].CYTHON, "oracle/_ref was not built (make -C oracle)"
+    cases["mas_cfg4"] = {"path": fixtures.record(R["helpers"].maximum_path(v, mask))}
+
+    torch.manual_seed(4)
+    pe = R["networks"].PosteriorEncoder(513, 192, 192, 5, 1, 16, cond_channels=256).eval()
+    c = {"posterior": _regenerate(pe, 5000)}
+    torch.manual_seed(14)
+    y, g = torch.randn(2, 513, 33).abs(), torch.randn(2, 256, 1)
+    lens = torch.tensor([33, 12])
+    torch.manual_seed(5)           # PosteriorEncoder draws randn_like(mean) inside forward (networks.py:287)
+    ref = pe(y, lens, g=g)
+    c["posterior_out"] = [fixtures.record(t) for t in ref]
+    fl = R["networks"].ResidualCouplingBlocks(192, 192, 5, 1, 4, cond_channels=256).eval()
+    perturb_zero_params(fl)
+    c["flow"] = _regenerate(fl, 6000)
+    c["flow_out"] = fixtures.record(fl(ref[0], ref[3], g=g))
+    dp = R["duration_predictor"].DurationPredictor(192, 256, 3, 0.5, cond_channels=256).eval()
+    c["dp"] = _regenerate(dp, 7000)
+    torch.manual_seed(15)
+    x = torch.randn(2, 192, 17)
+    xm = seq_mask(torch.tensor([17, 6]), 17)
+    c["dp_out"] = fixtures.record(dp(x, xm, g=g))
+    cases["voice_conversion_stack"] = c
+
+    def keys(m):
+        return {k: tuple(v.shape) for k, v in m.state_dict().items()}
+
+    cases["state_dict_keys"] = {
+        "TextEncoder": keys(R["networks"].TextEncoder(50, 192, 192, 768, 2, 6, 3, 0.1, language_emb_dim=4)),
+        "ResidualCouplingBlocks": keys(R["networks"].ResidualCouplingBlocks(192, 192, 5, 1, 4, cond_channels=256)),
+        "PosteriorEncoder": keys(R["networks"].PosteriorEncoder(513, 192, 192, 5, 1, 16, cond_channels=256)),
+        "StochasticDurationPredictor": keys(R["sdp"].StochasticDurationPredictor(192, 192, 3, 0.5, 4, cond_channels=256,
+                                                                                 language_emb_dim=4)),
+        "DurationPredictor": keys(R["duration_predictor"].DurationPredictor(192, 256, 3, 0.5, cond_channels=256,
+                                                                            language_emb_dim=4)),
+        "HifiganGenerator": keys(R["hifigan"].HifiganGenerator(
+            in_channels=192, out_channels=1, resblock_type="1", resblock_dilation_sizes=[[1, 3, 5]] * 3,
+            resblock_kernel_sizes=[3, 7, 11], upsample_kernel_sizes=[16, 16, 4, 4], upsample_initial_channel=512,
+            upsample_factors=[8, 8, 2, 2], inference_padding=0, cond_channels=256, conv_pre_weight_norm=False,
+            conv_post_weight_norm=False, conv_post_bias=False)),
+    }
+    save("oracle_vs_reference_full_width", cases)
+
+
+def _perturb_seeded(m, seed=0):
+    gen = torch.Generator().manual_seed(seed)
+    for _, p in m.named_parameters():
+        if float(p.abs().sum()) == 0.0:
+            p.data.copy_(torch.randn(p.shape, generator=gen) * 0.05)
+
+
+@torch.no_grad()
+def main_real_model():
+    """The real Vits.inference / voice_conversion / forward_mas with a narrow decoder
+    (tests/test_oracle_vs_reference_model.py); the test replays the same random draws for the oracle."""
+    import dataclasses
+    import types
+    F = ref_import.load_full()
+    base = dict(upsample_initial_channel_decoder=64, num_layers_text_encoder=2, hidden_channels_ffn_text_encoder=256)
+    cases = {}
+
+    def run(name, b, t, lens, seed, model_args=None, aux_extra=None, audio_sample_rate=None, attrs=None,
+            language_manager=None):
+        args = F["vits_model"].VitsArgs(**{**base, **(model_args or {})})
+        cfg = F["vits_config"].VitsConfig()
+        cfg.model_args = args
+        cfg.__post_init__()
+        if audio_sample_rate:
+            cfg.audio.sample_rate = audio_sample_rate
+        torch.manual_seed(seed)
+        m = F["vits_model"].Vits(cfg, language_manager=language_manager).eval()
+        _perturb_seeded(m, seed)
+        for k, v in (attrs or {}).items():
+            setattr(m, k, v)
+        c = _regenerate(m, 100000 * seed)
+        torch.manual_seed(seed + 100)
+        tok = torch.randint(0, args.num_chars, (b, t))
+        aux = {"x_lengths": lens, "d_vectors": None, "speaker_ids": None, "language_ids": None, "durations": None}
+        aux.update(aux_extra or {})
+        torch.manual_seed(seed + 1)
+        want = m.inference(tok, aux_input=dict(aux))
+        a = dataclasses.asdict(args)
+        a["length_scale"] = m.length_scale
+        a["max_inference_len"] = m.max_inference_len
+        a["sample_rate"] = cfg.audio.sample_rate
+        c.update({"args": a, "b": b, "t": t, "x_lengths": lens, "aux": aux_extra or {},
+                  "out": {k: fixtures.record(v) for k, v in want.items()}})
+        cases[name] = c
+
+    run("single_speaker", 3, 17, torch.tensor([17, 9, 4]), 3)
+    run("speaker_embedding_and_length_scale", 3, 12, torch.tensor([12, 7, 3]), 4,
+        dict(use_speaker_embedding=True, num_speakers=11), {"speaker_ids": torch.tensor([10, 0, 4])},
+        attrs={"length_scale": 1.6})
+    torch.manual_seed(50)
+    run("d_vectors", 2, 10, torch.tensor([10, 6]), 5, dict(use_d_vector_file=True, d_vector_dim=32),
+        {"d_vectors": torch.randn(2, 32)})
+    run("language_embedding", 2, 9, torch.tensor([9, 5]), 6,
+        dict(use_language_embedding=True, num_languages=3, embedded_language_dim=4), {"language_ids": torch.tensor([2, 0])},
+        language_manager=types.SimpleNamespace(num_languages=3))   # sizes emb_l like the LanguageManager (vits.py:795-799)
+    run("deterministic_dp_and_max_inference_len", 2, 11, torch.tensor([11, 6]), 7,
+        dict(use_sdp=False, use_speaker_embedding=True, num_speakers=4), {"speaker_ids": torch.tensor([1, 3])},
+        attrs={"max_inference_len": 9})
+    run("encoder_sample_rate", 2, 8, torch.tensor([8, 3]), 8,
+        dict(encoder_sample_rate=11025, upsample_rates_decoder=[8, 8, 4, 2], upsample_kernel_sizes_decoder=[16, 16, 8, 4]),
+        audio_sample_rate=22050)
+
+    args = F["vits_model"].VitsArgs(**base, use_speaker_embedding=True, num_speakers=5)
+    cfg = F["vits_config"].VitsConfig()
+    cfg.model_args = args
+    cfg.__post_init__()
+    torch.manual_seed(9)
+    m = F["vits_model"].Vits(cfg).eval()
+    _perturb_seeded(m, 9)
+    c = _regenerate(m, 900000)
+    torch.manual_seed(19)
+    y = torch.rand(1, 513, 14)
+    torch.manual_seed(10)          # PosteriorEncoder: torch.randn_like(mean), networks.py:287
+    o_hat, y_mask, (z, z_p, z_hat) = m.voice_conversion(y, torch.tensor([14]), 1, 4)
+    c.update({"args": dataclasses.asdict(args), "out": [fixtures.record(t) for t in (o_hat, y_mask, z, z_p, z_hat)]})
+    cases["voice_conversion"] = c
+
+    args = F["vits_model"].VitsArgs(**base)
+    cfg = F["vits_config"].VitsConfig()
+    cfg.model_args = args
+    cfg.__post_init__()
+    torch.manual_seed(12)
+    m = F["vits_model"].Vits(cfg).train()
+    b, ch, tx, ty = 3, 192, 11, 47
+    x_mask = seq_mask(torch.tensor([11, 7, 4]), tx)
+    y_mask = seq_mask(torch.tensor([47, 30, 21]), ty)
+    torch.manual_seed(13)
+    z_p, m_p, logs_p = torch.randn(b, ch, ty), torch.randn(b, ch, tx), torch.randn(b, ch, tx) * 0.3
+    x = torch.randn(b, ch, tx)
+    _, attn = m.forward_mas({}, z_p, m_p, logs_p, x, x_mask, y_mask, g=None, lang_emb=None)
+    cases["forward_mas"] = {"attn": fixtures.record(attn)}
+    save("oracle_vs_reference_model", cases)
+
+
+@torch.no_grad()
+def main_reference_objects():
+    """Answers of the reference's tokenizer / vocabulary, fairseq re-keying and vocoder config objects
+    (tests/test_handoff_cpu.py)."""
+    F = ref_import.load_full()
+    vocab = list("_ abcdefghijklmnopqrstuvwxyz'!?") + ["<x>"]
+    ref_v = F["characters"].BaseVocabulary(vocab, pad="_", blank=None, bos=None, eos=None)
+    out = {"vocab": vocab, "ids": {n: getattr(ref_v, n) for n in ("pad_id", "blank_id", "bos_id", "eos_id", "num_chars")}}
+    texts = ("What's  up?", "", "UPPER lower", "x")
+    tok = {}
+    for add_blank in (False, True):
+        t = F["tokenizer"].TTSTokenizer(False, F["cleaners"].basic_cleaners, ref_v, None, add_blank=add_blank)
+        tok[add_blank] = {"text_to_ids": [t.text_to_ids(x) for x in texts],
+                          "intersperse_blank": t.intersperse_blank_char([1, 2, 3], True),
+                          "intersperse_no_blank": t.intersperse_blank_char([1, 2], False),
+                          "pad_with_bos_eos": t.pad_with_bos_eos([4, 5])}
+    out.update({"texts": list(texts), "tokenizer": [tok[False], tok[True]]})
+
+    import tempfile
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_handoff_cpu import _fake_fairseq_state
+    with tempfile.TemporaryDirectory() as d:
+        p = os.path.join(d, "G_100000.pth")
+        torch.save({"model": _fake_fairseq_state()}, p)
+        out["fairseq"] = F["fairseq"].rehash_fairseq_vits_checkpoint(p)
+
+    rc = F["hifigan_config"].HifiganConfig()
+    ref_g = F["vocoder_models"].setup_generator(rc)
+    ra = rc.audio
+    out["hifigan_config"] = {
+        "generator_model": rc.generator_model, "generator_model_params": rc.generator_model_params,
+        "generator_state": [(k, tuple(v.shape)) for k, v in ref_g.state_dict().items()],
+        "audio": {f: getattr(ra, f) for f in ("fft_size", "win_length", "hop_length", "sample_rate", "num_mels",
+                                              "ref_level_db", "min_level_db", "signal_norm", "symmetric_norm",
+                                              "max_norm", "clip_norm")}}
+    save("reference_objects", out)
 
 
 if __name__ == "__main__":

@@ -1,15 +1,18 @@
 """Host-side widening of the path (SURVEY 8 f3 / f4), CPU only: tokenizer hand-off, fairseq checkpoint re-keying,
 HifiganConfig / setup_generator / GAN surface, and the oracle's restated vocoder hand-off -- each against the committed
-golden vectors (produced by the real reference, tests/golden/make_golden.py) and, where /root/reference exists,
-against the reference objects themselves."""
+golden vectors (produced by the real reference, tests/golden/make_golden.py), including the recorded answers of the
+reference objects themselves (tests/golden/reference_objects.pt)."""
 import numpy as np
 import pytest
 import torch
 
-import ref_import
+import fixtures
 import vits_oracle as O
 
-HAVE_REF = ref_import.available()
+
+@pytest.fixture(autouse=True)
+def _recorded_threads():
+    yield from fixtures.recorded_threads()
 
 
 # ----------------------------------------------------------------------------- tokenizer
@@ -37,23 +40,18 @@ def test_tokenizer_matches_reference_golden(golden, capsys):
     assert "ü" in tok.not_found_characters or tok.text_to_ids("ü") == [tok.characters.blank_id]   # unknown chars are dropped
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
-def test_tokenizer_and_vocabulary_vs_reference_objects(capsys):
+def test_tokenizer_and_vocabulary_vs_reference_objects(golden, capsys):
     from tts_b200.text import BaseVocabulary, TTSTokenizer, basic_cleaners
-    R = ref_import.load_full()
-    vocab = list("_ abcdefghijklmnopqrstuvwxyz'!?") + ["<x>"]
-    ref_v = R["characters"].BaseVocabulary(vocab, pad="_", blank=None, bos=None, eos=None)
-    my_v = BaseVocabulary(vocab, pad="_")
-    for name in ("pad_id", "blank_id", "bos_id", "eos_id", "num_chars"):
-        assert getattr(ref_v, name) == getattr(my_v, name)
-    for add_blank in (False, True):
-        ref_t = R["tokenizer"].TTSTokenizer(False, R["cleaners"].basic_cleaners, ref_v, None, add_blank=add_blank)
+    ref = golden("reference_objects")
+    my_v = BaseVocabulary(ref["vocab"], pad="_")
+    for name, want in ref["ids"].items():
+        assert getattr(my_v, name) == want, name
+    for add_blank, want in zip((False, True), ref["tokenizer"]):
         my_t = TTSTokenizer(False, basic_cleaners, my_v, None, add_blank=add_blank)
-        for text in ("What's  up?", "", "UPPER lower", "x"):
-            assert ref_t.text_to_ids(text) == my_t.text_to_ids(text)
-            assert ref_t.intersperse_blank_char([1, 2, 3], True) == my_t.intersperse_blank_char([1, 2, 3], True)
-            assert ref_t.intersperse_blank_char([1, 2], False) == my_t.intersperse_blank_char([1, 2], False)
-            assert ref_t.pad_with_bos_eos([4, 5]) == my_t.pad_with_bos_eos([4, 5])
+        assert [my_t.text_to_ids(text) for text in ref["texts"]] == want["text_to_ids"]
+        assert my_t.intersperse_blank_char([1, 2, 3], True) == want["intersperse_blank"]
+        assert my_t.intersperse_blank_char([1, 2], False) == want["intersperse_no_blank"]
+        assert my_t.pad_with_bos_eos([4, 5]) == want["pad_with_bos_eos"]
     capsys.readouterr()
 
 
@@ -68,7 +66,7 @@ def _fake_fairseq_state():
     return {k: torch.full((1,), float(i)) for i, k in enumerate(keys)}
 
 
-def test_fairseq_rekeying(tmp_path):
+def test_fairseq_rekeying(tmp_path, golden):
     from tts_b200.text import rehash_fairseq_vits_checkpoint
     sd = _fake_fairseq_state()
     p = tmp_path / "G_100000.pth"
@@ -87,11 +85,10 @@ def test_fairseq_rekeying(tmp_path):
     for old, new in want_names.items():
         assert new in got and torch.equal(got[new], sd[old]), (old, new)
     assert len(got) == len(sd)
-    if HAVE_REF:
-        ref = ref_import.load_full()["fairseq"].rehash_fairseq_vits_checkpoint(str(p))
-        assert set(ref.keys()) == set(got.keys())
-        for k in ref:
-            assert torch.equal(ref[k], got[k])
+    ref = golden("reference_objects")["fairseq"]
+    assert set(ref.keys()) == set(got.keys())
+    for k in ref:
+        assert torch.equal(ref[k], got[k])
 
 
 def test_fairseq_vocab_and_tokenizer(tmp_path):
@@ -105,7 +102,7 @@ def test_fairseq_vocab_and_tokenizer(tmp_path):
 
 
 # ----------------------------------------------------------------------------- vocoder config surface
-def test_hifigan_config_and_setup_generator_surface():
+def test_hifigan_config_and_setup_generator_surface(golden):
     from tts_b200.vocoder import GAN, BaseAudioConfig, HifiganConfig, setup_generator, to_camel
     c = HifiganConfig()
     assert c.generator_model == "hifigan_generator" and c["generator_model_params"]["upsample_factors"] == [8, 8, 2, 2]
@@ -117,17 +114,11 @@ def test_hifigan_config_and_setup_generator_surface():
     assert set(k.split(".")[0] for k in gan.state_dict()) == {"model_g"}
     with pytest.raises(NotImplementedError):
         setup_generator(HifiganConfig(generator_model="melgan_generator"))
-    if HAVE_REF:
-        R = ref_import.load_full()
-        rc = R["hifigan_config"].HifiganConfig()
-        assert rc.generator_model_params == c.generator_model_params and rc.generator_model == c.generator_model
-        ref_g = R["vocoder_models"].setup_generator(rc)
-        assert list(ref_g.state_dict().keys()) == list(g.state_dict().keys())
-        assert [tuple(v.shape) for v in ref_g.state_dict().values()] == [tuple(v.shape) for v in g.state_dict().values()]
-        ra = rc.audio
-        for f in ("fft_size", "win_length", "hop_length", "sample_rate", "num_mels", "ref_level_db", "min_level_db",
-                  "signal_norm", "symmetric_norm", "max_norm", "clip_norm"):
-            assert getattr(BaseAudioConfig(), f) == getattr(ra, f), f
+    rc = golden("reference_objects")["hifigan_config"]
+    assert rc["generator_model_params"] == c.generator_model_params and rc["generator_model"] == c.generator_model
+    assert rc["generator_state"] == [(k, tuple(v.shape)) for k, v in g.state_dict().items()]
+    for f, want in rc["audio"].items():
+        assert getattr(BaseAudioConfig(), f) == want, f
 
 
 # ----------------------------------------------------------------------------- oracle hand-off vs golden / reference

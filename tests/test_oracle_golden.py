@@ -1,9 +1,16 @@
 """Pins oracle/vits_oracle.py (+ the C MAS port) against fixtures produced by the unmodified reference
 (tests/golden/make_golden.py).  Bit-exact on CPU: the oracle issues the same torch ops."""
 import numpy as np
+import pytest
 import torch
 
+import fixtures
 import vits_oracle as O
+
+
+@pytest.fixture(autouse=True)
+def _recorded_threads():
+    yield from fixtures.recorded_threads()
 
 
 def test_hifigan_v1_small(golden):

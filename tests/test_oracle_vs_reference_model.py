@@ -1,161 +1,100 @@
 """Pins the oracle's restated ``Vits.inference`` glue (oracle/vits_oracle.py: vits_inference, voice_conversion) against
-the REAL, unmodified reference model class ``TTS.tts.models.vits.Vits`` -- importable in the build container once inert
-placeholders stand in for the third-party packages that are not installed (oracle/ref_import.py).  Round 1 could only
-pin the layer modules and had to restate the glue unpinned; this closes that gap: same weights, same random draws,
-``torch.equal`` on every output of the reference's 8-key dict.
-
-Skipped where /root/reference is absent (the GPU box)."""
-import dataclasses
-
+the REAL, unmodified reference model class ``TTS.tts.models.vits.Vits``: same weights, same random draws,
+``torch.equal`` on every output of the reference's 8-key dict.  The reference's answers come from the compact fixture
+tests/golden/oracle_vs_reference_model.pt (tests/golden/make_golden.py; oracle/fixtures.py says what is stored)."""
 import pytest
 import torch
 
-import ref_import
+import fixtures
 import vits_oracle as O
-
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
-
-
-@pytest.fixture(scope="module")
-def R():
-    return ref_import.load_full()
+from fixtures import check, state_from_stats
 
 
-def _perturb(m, seed=0):
-    gen = torch.Generator().manual_seed(seed)
-    for _, p in m.named_parameters():
-        if float(p.abs().sum()) == 0.0:
-            p.data.copy_(torch.randn(p.shape, generator=gen) * 0.05)
+@pytest.fixture(autouse=True)
+def _recorded_threads():
+    yield from fixtures.recorded_threads()
 
 
-def _small_args(R, **kw):
-    # narrow decoder so the CPU run takes seconds; every code path of the glue is unchanged
-    base = dict(upsample_initial_channel_decoder=64, num_layers_text_encoder=2, hidden_channels_ffn_text_encoder=256)
-    base.update(kw)
-    return R["vits_model"].VitsArgs(**base)
+KEYS = ("model_outputs", "alignments", "durations", "z", "z_p", "m_p", "logs_p", "y_mask")
 
 
-def _run_both(R, args, b, t, lens, seed, aux_extra=None, audio_sample_rate=None, attrs=None, language_manager=None):
-    cfg = R["vits_config"].VitsConfig()
-    cfg.model_args = args
-    cfg.__post_init__()
-    if audio_sample_rate:
-        cfg.audio.sample_rate = audio_sample_rate
-    torch.manual_seed(seed)
-    m = R["vits_model"].Vits(cfg, language_manager=language_manager).eval()
-    _perturb(m, seed)
-    for k, v in (attrs or {}).items():
-        setattr(m, k, v)
-    tok = torch.randint(0, args.num_chars, (b, t))
-    aux = {"x_lengths": lens, "d_vectors": None, "speaker_ids": None, "language_ids": None, "durations": None}
-    aux.update(aux_extra or {})
-    torch.manual_seed(seed + 1)
-    want = m.inference(tok, aux_input=dict(aux))
+def _run(golden, name, seed):
+    c = golden("oracle_vs_reference_model")[name]
+    a, b, t = c["args"], c["b"], c["t"]
+    torch.manual_seed(seed + 100)
+    tok = torch.randint(0, a["num_chars"], (b, t))
     # the reference draws the SDP noise first (stochastic_duration_predictor.py:287, CPU generator), then
     # randn_like(m_p) (vits.py:1155): replay the same stream for the oracle
     torch.manual_seed(seed + 1)
-    sdp_noise = torch.randn(b, 2, t) if args.use_sdp else None
-    a = dataclasses.asdict(args)
-    a["length_scale"] = m.length_scale
-    a["max_inference_len"] = m.max_inference_len
-    a["sample_rate"] = cfg.audio.sample_rate
+    sdp_noise = torch.randn(b, 2, t) if a["use_sdp"] else None
     # m_p is a transposed view there ([B,T,C] storage seen as [B,C,T]); randn_like keeps the strides and a non-contiguous
     # CPU normal_() takes the serial sampler, not the vectorised fill: replay with the same call on the same layout
-    got = O.vits_inference(m.state_dict(), tok, lens, sdp_noise,
+    got = O.vits_inference(state_from_stats(c["stats"], c["seed"]), tok, c["x_lengths"], sdp_noise,
                            lambda s: torch.randn_like(torch.empty(s[0], s[2], s[1]).transpose(1, 2)), args=a,
-                           speaker_ids=aux.get("speaker_ids"), d_vectors=aux.get("d_vectors"),
-                           language_ids=aux.get("language_ids"))
-    for k in ("model_outputs", "alignments", "durations", "z", "z_p", "m_p", "logs_p", "y_mask"):
-        assert got[k].shape == want[k].shape, (k, got[k].shape, want[k].shape)
-        assert torch.equal(got[k], want[k]), k
-    return want
+                           speaker_ids=c["aux"].get("speaker_ids"), d_vectors=c["aux"].get("d_vectors"),
+                           language_ids=c["aux"].get("language_ids"))
+    assert set(c["out"]) == set(KEYS)
+    for k in KEYS:
+        check(got[k], c["out"][k], k)
+    return got
 
 
 @torch.no_grad()
-def test_single_speaker_glue_bit_exact(R):
-    out = _run_both(R, _small_args(R), b=3, t=17, lens=torch.tensor([17, 9, 4]), seed=3)
-    assert set(out.keys()) == {"model_outputs", "alignments", "durations", "z", "z_p", "m_p", "logs_p", "y_mask"}
+def test_single_speaker_glue_bit_exact(golden):
+    out = _run(golden, "single_speaker", 3)
     assert out["model_outputs"].shape[-1] == out["y_mask"].shape[-1] * 256
 
 
 @torch.no_grad()
-def test_speaker_embedding_and_length_scale(R):
-    args = _small_args(R, use_speaker_embedding=True, num_speakers=11)
-    _run_both(R, args, b=3, t=12, lens=torch.tensor([12, 7, 3]), seed=4,
-              aux_extra={"speaker_ids": torch.tensor([10, 0, 4])}, attrs={"length_scale": 1.6})
+def test_speaker_embedding_and_length_scale(golden):
+    _run(golden, "speaker_embedding_and_length_scale", 4)
 
 
 @torch.no_grad()
-def test_d_vectors(R):
-    args = _small_args(R, use_d_vector_file=True, d_vector_dim=32)
-    _run_both(R, args, b=2, t=10, lens=torch.tensor([10, 6]), seed=5, aux_extra={"d_vectors": torch.randn(2, 32)})
+def test_d_vectors(golden):
+    _run(golden, "d_vectors", 5)
 
 
 @torch.no_grad()
-def test_language_embedding(R):
-    args = _small_args(R, use_language_embedding=True, num_languages=3, embedded_language_dim=4)
-    import types
-    lm = types.SimpleNamespace(num_languages=3)      # the reference sizes emb_l from its LanguageManager (vits.py:795-799)
-    _run_both(R, args, b=2, t=9, lens=torch.tensor([9, 5]), seed=6, aux_extra={"language_ids": torch.tensor([2, 0])},
-              language_manager=lm)
+def test_language_embedding(golden):
+    _run(golden, "language_embedding", 6)
 
 
 @torch.no_grad()
-def test_deterministic_duration_predictor_and_max_inference_len(R):
-    args = _small_args(R, use_sdp=False, use_speaker_embedding=True, num_speakers=4)
-    _run_both(R, args, b=2, t=11, lens=torch.tensor([11, 6]), seed=7, aux_extra={"speaker_ids": torch.tensor([1, 3])},
-              attrs={"max_inference_len": 9})
+def test_deterministic_duration_predictor_and_max_inference_len(golden):
+    _run(golden, "deterministic_dp_and_max_inference_len", 7)
 
 
 @torch.no_grad()
-def test_encoder_sample_rate_upsampling(R):
-    args = _small_args(R, encoder_sample_rate=11025, upsample_rates_decoder=[8, 8, 4, 2],
-                       upsample_kernel_sizes_decoder=[16, 16, 8, 4])
-    _run_both(R, args, b=2, t=8, lens=torch.tensor([8, 3]), seed=8, audio_sample_rate=22050)
+def test_encoder_sample_rate_upsampling(golden):
+    _run(golden, "encoder_sample_rate", 8)
 
 
 @torch.no_grad()
-def test_voice_conversion_glue_bit_exact(R):
-    args = _small_args(R, use_speaker_embedding=True, num_speakers=5)
-    cfg = R["vits_config"].VitsConfig()
-    cfg.model_args = args
-    cfg.__post_init__()
-    torch.manual_seed(9)
-    m = R["vits_model"].Vits(cfg).eval()
-    _perturb(m, 9)
-    # the reference embeds `speaker_cond` as emb_g(tensor(id).unsqueeze(0)) (vits.py:1216-1217): one utterance, scalar ids
+def test_voice_conversion_glue_bit_exact(golden):
+    c = golden("oracle_vs_reference_model")["voice_conversion"]
+    torch.manual_seed(19)
     y = torch.rand(1, 513, 14)
-    lens = torch.tensor([14])
-    src, tgt = 1, 4
-    torch.manual_seed(10)
-    o_hat, y_mask, (z, z_p, z_hat) = m.voice_conversion(y, lens, src, tgt)
     torch.manual_seed(10)
     noise = torch.randn(1, 192, 14)       # PosteriorEncoder: torch.randn_like(mean), networks.py:287
-    sd = m.state_dict()
+    sd = state_from_stats(c["stats"], c["seed"])
+    # the reference embeds `speaker_cond` as emb_g(tensor(id).unsqueeze(0)) (vits.py:1216-1217): one utterance, scalar ids
     g = lambda i: torch.nn.functional.embedding(torch.tensor([i]), sd["emb_g.weight"]).unsqueeze(-1)
-    go, gm, (gz, gzp, gzh) = O.voice_conversion(sd, y, lens, g(src), g(tgt), noise, args=dataclasses.asdict(args))
-    for a, b in ((go, o_hat), (gm, y_mask), (gz, z), (gzp, z_p), (gzh, z_hat)):
-        assert torch.equal(a, b)
+    go, gm, (gz, gzp, gzh) = O.voice_conversion(sd, y, torch.tensor([14]), g(1), g(4), noise, args=c["args"])
+    for i, a in enumerate((go, gm, gz, gzp, gzh)):
+        check(a, c["out"][i], ("o_hat", "y_mask", "z", "z_p", "z_hat")[i])
 
 
 @torch.no_grad()
-def test_forward_mas_alignment_vs_real_model(R):
+def test_forward_mas_alignment_vs_real_model(golden):
     """Vits.forward_mas (vits.py:909-919) on the real model class: the oracle's logp / attn restatement is bit-exact
-    (the real maximum_path runs the reference's compiled Cython kernel)."""
-    args = _small_args(R)
-    cfg = R["vits_config"].VitsConfig()
-    cfg.model_args = args
-    cfg.__post_init__()
-    torch.manual_seed(12)
-    m = R["vits_model"].Vits(cfg).train()
+    (the real maximum_path ran the reference's compiled Cython kernel)."""
+    want = golden("oracle_vs_reference_model")["forward_mas"]["attn"]
     b, c, tx, ty = 3, 192, 11, 47
-    xl, yl = torch.tensor([11, 7, 4]), torch.tensor([47, 30, 21])
-    x_mask = O.sequence_mask(xl, tx).unsqueeze(1).float()
-    y_mask = O.sequence_mask(yl, ty).unsqueeze(1).float()
+    x_mask = O.sequence_mask(torch.tensor([11, 7, 4]), tx).unsqueeze(1).float()
+    y_mask = O.sequence_mask(torch.tensor([47, 30, 21]), ty).unsqueeze(1).float()
+    torch.manual_seed(13)
     z_p, m_p, logs_p = torch.randn(b, c, ty), torch.randn(b, c, tx), torch.randn(b, c, tx) * 0.3
-    x = torch.randn(b, c, tx)
-    outputs, attn = m.forward_mas({}, z_p, m_p, logs_p, x, x_mask, y_mask, g=None, lang_emb=None)
-    got, _ = O.forward_mas_attn(z_p, m_p, logs_p, x_mask, y_mask, impl="ref")
-    assert torch.equal(got, attn)
-    got_c, _ = O.forward_mas_attn(z_p, m_p, logs_p, x_mask, y_mask, impl="c")
-    assert torch.equal(got_c, attn)
+    for impl in ("c", "py"):
+        got, _ = O.forward_mas_attn(z_p, m_p, logs_p, x_mask, y_mask, impl=impl)
+        check(got, want, impl)
