@@ -26,6 +26,22 @@
 extern "C" {
 #endif
 
+/* Numerical precision of the tensor-core conv layers (the `precision` argument of the *_create_ex calls).
+ *   B200TTS_PRECISION_FP32 (the default of every other create call): 3xTF32.  Both operands are split into
+ *     hi + lo TF32 parts and each tap issues lo*hi + hi*lo + hi*hi, accumulated in fp32: within ~1e-5 relative RMS of
+ *     an fp32 computation per layer, and the HiFiGAN waveform within 1e-4 RMS of the fp32 reference.
+ *   B200TTS_PRECISION_TF32: single-pass TF32, the numerics PyTorch's cuDNN convolutions use by default
+ *     (torch.backends.cudnn.allow_tf32).  Activations (after the leaky ReLU) and weights are rounded to TF32 -- to
+ *     nearest, ties away from zero -- and each tap is one MMA accumulated in fp32.  Per output element the error is
+ *     at most about (2^-10 + Cin*K*2^-23) * sum|w||x| plus the fp32 epilogue's roundings; measured on a B200:
+ *     1e-4 to 3e-4 relative RMS per layer, 2e-4 to 5e-4 on the HiFiGAN waveform (cuDNN's TF32 on the same inputs:
+ *     about 8e-4).  Faster: a third of the MMAs and of the operand bytes in shared memory, half the weight bytes.
+ * Layers that do not run on the tensor cores (HiFiGAN conv_post and cond_layer, anything narrower than 32 rows, and
+ * every layer created with allow_tensor_cores = 0) are exact FP32 in both modes.  Results are deterministic in both:
+ * identical calls give identical bits, and a ragged call equals the dense one on every valid sample. */
+#define B200TTS_PRECISION_FP32 0
+#define B200TTS_PRECISION_TF32 1
+
 const char* b200tts_last_error(void);
 /* number of kernels launched by this library in this process (bench.py "gpu_launches") */
 unsigned long long b200tts_launch_count(void);
@@ -37,7 +53,8 @@ int b200tts_debug_tc_error(void);
 
 /* Debug / test aids: record, on the calling thread, which kernel family every conv launch dispatched to.
  * ids: 0 FP32-FMA tile kernel, 1 tcgen05 v1, 2 tcgen05 v2 (M = time), 3 tcgen05 v3 (M = rows), 4 v3 + staged epilogue,
- *      5 v3 grouped (narrow layers), 6 single-row streaming kernel (conv_post), 7 fused ResBlock kernel. */
+ *      5 v3 grouped (narrow layers), 6 single-row streaming kernel (conv_post), 7 fused ResBlock kernel,
+ *      8 v3 single-pass TF32, 9 v3 grouped single-pass TF32. */
 void b200tts_debug_dispatch_begin(void);
 int b200tts_debug_dispatch_end(int32_t* ids, int cap); /* returns the number of launches recorded */
 
@@ -59,6 +76,10 @@ typedef struct {
 typedef struct b200tts_conv1d b200tts_conv1d;
 int b200tts_conv1d_create(const b200tts_conv1d_config* cfg, const float* weight, const float* bias,
                           int allow_tensor_cores, b200tts_conv1d** out);
+/* the same with an explicit B200TTS_PRECISION_* for the tensor-core kernels (b200tts_conv1d_create = FP32);
+ * an unknown precision returns 1 */
+int b200tts_conv1d_create_ex(const b200tts_conv1d_config* cfg, const float* weight, const float* bias,
+                             int allow_tensor_cores, int precision, b200tts_conv1d** out);
 void b200tts_conv1d_destroy(b200tts_conv1d* h);
 int b200tts_conv1d_out_len(const b200tts_conv1d* h, int T);
 int b200tts_conv1d_forward(const b200tts_conv1d* h, const float* x, int B, int T, float in_slope, const float* residual,
@@ -117,6 +138,12 @@ typedef struct {
 typedef struct b200tts_hifigan b200tts_hifigan;
 int b200tts_hifigan_create(const b200tts_hifigan_config* cfg, const float* const* weights, int num_weights,
                            b200tts_hifigan** out);
+/* the same with an explicit B200TTS_PRECISION_* for conv_pre, the upsamplers and the ResBlock convs
+ * (b200tts_hifigan_create = FP32); an unknown precision returns 1.  b200tts_hifigan_precision: the handle's mode
+ * (-1 for NULL). */
+int b200tts_hifigan_create_ex(const b200tts_hifigan_config* cfg, const float* const* weights, int num_weights,
+                              int precision, b200tts_hifigan** out);
+int b200tts_hifigan_precision(const b200tts_hifigan* h);
 void b200tts_hifigan_destroy(b200tts_hifigan* h);
 size_t b200tts_hifigan_workspace_bytes(const b200tts_hifigan* h, int B, int T);
 int b200tts_hifigan_out_len(const b200tts_hifigan* h, int T);

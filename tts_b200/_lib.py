@@ -68,7 +68,19 @@ class AudioNormC(ctypes.Structure):
                 ("scaler_mean", ctypes.c_void_p), ("scaler_scale", ctypes.c_void_p)]
 
 
-DISPATCH_NAMES = {0: "fma", 1: "tc1", 2: "tc2", 3: "tc3", 4: "tc3_staged", 5: "tc3_grouped", 6: "row1", 7: "resblock"}
+DISPATCH_NAMES = {0: "fma", 1: "tc1", 2: "tc2", 3: "tc3", 4: "tc3_staged", 5: "tc3_grouped", 6: "row1", 7: "resblock",
+                  8: "tc3_tf32", 9: "tc3_grouped_tf32"}
+
+# B200TTS_PRECISION_* of include/tts_b200.h: numerics of the tensor-core conv layers
+PRECISIONS = {"fp32": 0, "tf32": 1}
+
+
+def precision_id(precision):
+    """``"fp32"`` (3xTF32, the default) or ``"tf32"`` (single-pass TF32) -> the C ABI constant; anything else raises.
+    Pure Python: validating a setting needs no CUDA library."""
+    if not isinstance(precision, str) or precision not in PRECISIONS:
+        raise ValueError(f"tts_b200: precision must be one of {sorted(PRECISIONS)}, got {precision!r}")
+    return PRECISIONS[precision]
 
 
 def _declare(lib):
@@ -82,6 +94,8 @@ def _declare(lib):
     lib.b200tts_debug_dispatch_end.argtypes = [vp, ci]
     lib.b200tts_conv1d_create.restype = ci
     lib.b200tts_conv1d_create.argtypes = [ctypes.POINTER(Conv1dConfigC), vp, vp, ci, ctypes.POINTER(vp)]
+    lib.b200tts_conv1d_create_ex.restype = ci
+    lib.b200tts_conv1d_create_ex.argtypes = [ctypes.POINTER(Conv1dConfigC), vp, vp, ci, ci, ctypes.POINTER(vp)]
     lib.b200tts_conv1d_destroy.restype = None
     lib.b200tts_conv1d_destroy.argtypes = [vp]
     lib.b200tts_conv1d_out_len.restype = ci
@@ -114,6 +128,11 @@ def _declare(lib):
     lib.b200tts_hifigan_create.restype = ci
     lib.b200tts_hifigan_create.argtypes = [ctypes.POINTER(HifiganConfigC), ctypes.POINTER(vp), ci,
                                            ctypes.POINTER(vp)]
+    lib.b200tts_hifigan_create_ex.restype = ci
+    lib.b200tts_hifigan_create_ex.argtypes = [ctypes.POINTER(HifiganConfigC), ctypes.POINTER(vp), ci, ci,
+                                              ctypes.POINTER(vp)]
+    lib.b200tts_hifigan_precision.restype = ci
+    lib.b200tts_hifigan_precision.argtypes = [vp]
     lib.b200tts_hifigan_destroy.restype = None
     lib.b200tts_hifigan_destroy.argtypes = [vp]
     lib.b200tts_hifigan_workspace_bytes.restype = sz

@@ -15,13 +15,20 @@ from . import _lib
 
 class FusedConv1d:
     """weight [Cout,Cin,K] (or [Cin,Cout,K] with ``transposed=True``), bias [Cout] or None -- host or device tensors;
-    the packed device copy is created on first use per device."""
+    the packed device copy is created on first use per device.
 
-    def __init__(self, weight, bias=None, dilation=1, padding=0, transposed=False, stride=1, tensor_cores=True):
+    ``precision`` chooses the numerics of the tensor-core kernels: ``"fp32"`` (default, 3xTF32, within ~1e-5 relative
+    of fp32) or ``"tf32"`` (single-pass TF32 with round-to-nearest operands, cuDNN's default numerics; faster).  A layer
+    the tensor cores do not take (fewer than 32 output rows, ``tensor_cores=False``, ...) is exact FP32 either way."""
+
+    def __init__(self, weight, bias=None, dilation=1, padding=0, transposed=False, stride=1, tensor_cores=True,
+                 precision="fp32"):
         self.weight = weight.detach().to(torch.float32).cpu().contiguous()
         self.bias = None if bias is None else bias.detach().to(torch.float32).cpu().contiguous()
         self.dilation, self.padding, self.transposed, self.stride = int(dilation), int(padding), bool(transposed), int(stride)
         self.tensor_cores = bool(tensor_cores)
+        _lib.precision_id(precision)
+        self.precision = precision
         if transposed:
             self.cin, self.cout, self.k = self.weight.shape
         else:
@@ -41,8 +48,9 @@ class FusedConv1d:
             cfg = _lib.Conv1dConfigC(self.cin, self.cout, self.k, self.dilation, self.padding, int(self.transposed), self.stride)
             out = ctypes.c_void_p()
             with torch.cuda.device(device):
-                rc = _lib.lib().b200tts_conv1d_create(ctypes.byref(cfg), _lib.ptr(self.weight), _lib.ptr(self.bias),
-                                                      int(self.tensor_cores), ctypes.byref(out))
+                rc = _lib.lib().b200tts_conv1d_create_ex(ctypes.byref(cfg), _lib.ptr(self.weight), _lib.ptr(self.bias),
+                                                         int(self.tensor_cores), _lib.precision_id(self.precision),
+                                                         ctypes.byref(out))
             _lib.check(rc, "conv1d_create")
             self._handles[device] = h = out
         return h

@@ -17,25 +17,33 @@ extern "C" {
 
 const char* b200tts_last_error(void) { return last_error(); }
 unsigned long long b200tts_launch_count(void) { return g_launch_count; }
-int b200tts_version(void) { return 100; }
+int b200tts_version(void) { return 101; }
 int b200tts_debug_tc_error(void) { return conv_tc_error_flag(); }
 void b200tts_debug_dispatch_begin(void) { dispatch_begin(); }
 int b200tts_debug_dispatch_end(int32_t* ids, int cap) { return dispatch_end(ids, cap); }
 
 struct b200tts_conv1d { ConvLayer L; b200tts_conv1d_config c; ~b200tts_conv1d() { free_conv(L); } };
 
+static bool known_precision(int p) { return p == B200TTS_PRECISION_FP32 || p == B200TTS_PRECISION_TF32; }
+
 int b200tts_conv1d_create(const b200tts_conv1d_config* cfg, const float* weight, const float* bias, int allow_tensor_cores,
                           b200tts_conv1d** out) {
+    return b200tts_conv1d_create_ex(cfg, weight, bias, allow_tensor_cores, B200TTS_PRECISION_FP32, out);
+}
+int b200tts_conv1d_create_ex(const b200tts_conv1d_config* cfg, const float* weight, const float* bias, int allow_tensor_cores,
+                             int precision, b200tts_conv1d** out) {
     if (!cfg || !weight || !out) { set_error("conv1d_create: null argument"); return 1; }
     *out = nullptr;
+    if (!known_precision(precision)) { set_error("conv1d_create: unknown precision %d", precision); return 1; }
+    const int tp = precision == B200TTS_PRECISION_TF32 ? 1 : 3;
     b200tts_conv1d* h = new (std::nothrow) b200tts_conv1d();
     if (!h) { set_error("conv1d_create: out of host memory"); return 1; }
     h->c = *cfg;
     int rc = cfg->transposed
                  ? pack_conv_transpose(h->L, weight, bias, cfg->in_channels, cfg->out_channels, cfg->kernel_size,
-                                       cfg->stride, cfg->padding)
+                                       cfg->stride, cfg->padding, tp)
                  : pack_conv(h->L, weight, bias, cfg->out_channels, cfg->in_channels, cfg->kernel_size, cfg->dilation,
-                             cfg->padding);
+                             cfg->padding, 0, nullptr, nullptr, tp);
     if (rc) { delete h; return rc; }
     h->L.allow_tc = allow_tensor_cores != 0;
     *out = h;
@@ -78,15 +86,21 @@ int b200tts_mas_from_stats(const float* z_p, const float* m_p, const float* logs
 
 int b200tts_hifigan_create(const b200tts_hifigan_config* cfg, const float* const* weights, int num_weights,
                            b200tts_hifigan** out) {
+    return b200tts_hifigan_create_ex(cfg, weights, num_weights, B200TTS_PRECISION_FP32, out);
+}
+int b200tts_hifigan_create_ex(const b200tts_hifigan_config* cfg, const float* const* weights, int num_weights, int precision,
+                              b200tts_hifigan** out) {
     if (!cfg || !weights || !out) { set_error("hifigan_create: null argument"); return 1; }
     *out = nullptr;
+    if (!known_precision(precision)) { set_error("hifigan_create: unknown precision %d", precision); return 1; }
     b200tts_hifigan* h = new (std::nothrow) b200tts_hifigan();
     if (!h) { set_error("hifigan_create: out of host memory"); return 1; }
-    int rc = h->impl.init(*cfg, weights, num_weights);
+    int rc = h->impl.init(*cfg, weights, num_weights, precision);
     if (rc) { delete h; return rc; }
     *out = h;
     return 0;
 }
+int b200tts_hifigan_precision(const b200tts_hifigan* h) { return h ? h->impl.precision : -1; }
 void b200tts_hifigan_destroy(b200tts_hifigan* h) { delete h; }
 size_t b200tts_hifigan_workspace_bytes(const b200tts_hifigan* h, int B, int T) {
     return h ? h->impl.workspace_bytes(B, T) : 0;

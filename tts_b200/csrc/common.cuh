@@ -99,6 +99,8 @@ struct ConvLayer {            // immutable after pack(); owned by an engine hand
     int tc_grp = 0;           // tap groups of the grouped packing (128 / rows), 0: none
     bool allow_tc = false;    // engines opt layers into the 3xTF32 tensor-core path (decoder / flow); the text and
                               // duration path stays on the exact FP32 FMA kernel so durations remain bit-stable
+    int tc_passes = 3;        // how w_tc / w_tcg were packed: 3 (3xTF32, {hi,lo}) or 1 (single-pass TF32, rounded to
+                              // nearest); selects the matching tcgen05 kernels.  The FP32-FMA / single-row kernels ignore it
 };
 
 struct ConvIO {
@@ -128,16 +130,18 @@ struct ConvIO {
 // Host weights in PyTorch layout.  conv: w[Cout][Cin][K];  transposed: w[Cin][Cout][Kt].
 // gate_half > 0 interleaves rows (p, p+gate_half) for the fused WaveNet gate.
 // in_perm / out_perm (nullable) remap logical->physical channels (flow channel flips).
+// tc_passes: 3 (3xTF32) or 1 (single-pass TF32) for the tensor-core packings, see ConvLayer::tc_passes.
 int pack_conv(ConvLayer& L, const float* w, const float* bias, int Cout, int Cin, int K, int dil, int pad,
-              int gate_half = 0, const int* in_perm = nullptr, const int* out_perm = nullptr);
+              int gate_half = 0, const int* in_perm = nullptr, const int* out_perm = nullptr, int tc_passes = 3);
 int pack_conv_transpose(ConvLayer& L, const float* w, const float* bias, int Cin, int Cout, int Kt, int stride,
-                        int padding);
+                        int padding, int tc_passes = 3);
 void free_conv(ConvLayer& L);
 int launch_conv(const ConvLayer& L, const ConvIO& io, cudaStream_t stream);
 int conv_tc_error_flag();
 // which kernel family a launch_conv call dispatched to (recorded per thread between dispatch_begin/end; tests pin it)
 enum : int { DISPATCH_FMA = 0, DISPATCH_TC1 = 1, DISPATCH_TC2 = 2, DISPATCH_TC3 = 3, DISPATCH_TC3_STAGED = 4,
-             DISPATCH_TC3_GROUPED = 5, DISPATCH_ROW1 = 6, DISPATCH_RESBLOCK = 7 };
+             DISPATCH_TC3_GROUPED = 5, DISPATCH_ROW1 = 6, DISPATCH_RESBLOCK = 7, DISPATCH_TC3_TF32 = 8,
+             DISPATCH_TC3_GROUPED_TF32 = 9 };
 void dispatch_begin();
 int dispatch_end(int* ids, int cap);
 void dispatch_note(int id);

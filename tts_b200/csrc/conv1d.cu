@@ -412,9 +412,34 @@ void free_conv(ConvLayer& L) {
     L.w = L.bias = L.w_tc = L.w_tcg = nullptr;
 }
 
+// Host twin of the single-pass producers' cvt.rna.tf32.f32: round a finite value to the nearest TF32 value, ties away
+// from zero (sign-magnitude, so adding half an ulp to the bits and truncating does it); inf / NaN pass through.
+static float tf32_rna(float v) {
+    uint32_t u;
+    memcpy(&u, &v, 4);
+    if ((u & 0x7F800000u) != 0x7F800000u) { u += 0x1000u; u &= 0xFFFFE000u; }
+    memcpy(&v, &u, 4);
+    return v;
+}
+// One weight of a tcgen05 tap block: 3 passes -> hi (TF32 truncation) at hi[i], the exact remainder at lo[i];
+// 1 pass -> the TF32-rounded value at hi[i] (there is no lo half)
+static inline void put_tc_weight(float v, int passes, float* hi, float* lo, size_t i) {
+    if (passes == 1) { hi[i] = tf32_rna(v); return; }
+    uint32_t u;
+    memcpy(&u, &v, 4);
+    u &= 0xFFFFE000u;
+    float h;
+    memcpy(&h, &u, 4);
+    hi[i] = h;
+    lo[i] = v - h;
+}
+
 // Wl(r, ci, k): logical weights already expressed as a correlation-form conv with `rows` GEMM rows
 static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vector<float>& bl, int rows, int Cin,
-                     int K) {
+                     int K, int tc_passes) {
+    B200_REQUIRE(tc_passes == 1 || tc_passes == 3, "conv pack: tc_passes must be 1 or 3, got %d", tc_passes);
+    L.tc_passes = tc_passes;
+    const int halves = tc_passes == 1 ? 1 : 2;     // {hi, lo} or {w} per tap block
     L.Rows = rows;
     L.co_tile = rows >= 64 ? 64 : 32;
     L.RowsPad = round_up(rows, L.co_tile);
@@ -433,7 +458,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
     for (int r = 0; r < rows; ++r) bp[r] = bl[r];
     if (upload(&L.w, P.data(), P.size())) return 2;
     if (upload(&L.bias, bp.data(), bp.size())) return 2;
-    // tcgen05 packing (3xTF32 hi/lo split) for layers the tensor-core kernel can take
+    // tcgen05 packing (3xTF32 hi/lo split, or single-pass TF32) for layers the tensor-core kernel can take
     // rows >= 32: tiles of 128 zero-padded rows (tcgen05 M = 128); exactly 32 / 64 rows additionally get the grouped
     // packing below (no padding), which the dispatcher prefers; fewer rows run on the FP32-FMA kernel
     L.tc_n = 0;
@@ -441,7 +466,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
     if (L.tc_n && rows >= 16 && Cin >= 8) {
         using namespace tc;
         const int N = L.tc_n, nt = (rows + N - 1) / N, nchunk = (Cin + KC - 1) / KC;
-        const size_t blk = (size_t)2 * NSLAB * N * 4;
+        const size_t blk = (size_t)halves * NSLAB * N * 4;
         std::vector<float> Q((size_t)nt * nchunk * K * blk, 0.f);
         for (int tile = 0; tile < nt; ++tile)
             for (int c = 0; c < nchunk; ++c)
@@ -452,13 +477,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
                             for (int i = 0; i < 4; ++i) {
                                 const int r = tile * N + n, ci = c * KC + 4 * s2 + i;
                                 const float v = (ci < Cin && r < rows) ? Wl[((size_t)r * Cin + ci) * K + k] : 0.f;
-                                uint32_t u;
-                                memcpy(&u, &v, 4);
-                                u &= 0xFFFFE000u;
-                                float hi;
-                                memcpy(&hi, &u, 4);
-                                dst[((size_t)s2 * N + n) * 4 + i] = hi;
-                                dst[((size_t)(NSLAB + s2) * N + n) * 4 + i] = v - hi;
+                                put_tc_weight(v, tc_passes, dst, dst + (size_t)NSLAB * N * 4, ((size_t)s2 * N + n) * 4 + i);
                             }
                 }
         if (upload(&L.w_tc, Q.data(), Q.size())) return 2;
@@ -471,7 +490,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
     if (L.ups == 1 && (rows == 32 || rows == 64) && Cin >= 8) {
         using namespace tc;
         const int G = 128 / rows, J = (K + G - 1) / G, nchunk = (Cin + KC - 1) / KC;
-        const size_t blk = (size_t)2 * NSLAB * 128 * 4;
+        const size_t blk = (size_t)halves * NSLAB * 128 * 4;
         std::vector<float> Q((size_t)nchunk * J * blk, 0.f);
         for (int c = 0; c < nchunk; ++c)
             for (int j = 0; j < J; ++j) {
@@ -482,13 +501,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
                             const int g = m / rows, co = m % rows;
                             const int k = G * j + g, ci = c * KC + 4 * s2 + i;
                             const float v = (ci < Cin && k < K) ? Wl[((size_t)co * Cin + ci) * K + k] : 0.f;
-                            uint32_t u;
-                            memcpy(&u, &v, 4);
-                            u &= 0xFFFFE000u;
-                            float hi;
-                            memcpy(&hi, &u, 4);
-                            dst[((size_t)s2 * 128 + m) * 4 + i] = hi;
-                            dst[((size_t)(NSLAB + s2) * 128 + m) * 4 + i] = v - hi;
+                            put_tc_weight(v, tc_passes, dst, dst + (size_t)NSLAB * 128 * 4, ((size_t)s2 * 128 + m) * 4 + i);
                         }
             }
         if (upload(&L.w_tcg, Q.data(), Q.size())) return 2;
@@ -498,7 +511,7 @@ static int pack_rows(ConvLayer& L, const std::vector<float>& Wl, const std::vect
 }
 
 int pack_conv(ConvLayer& L, const float* w, const float* bias, int Cout, int Cin, int K, int dil, int pad,
-              int gate_half, const int* in_perm, const int* out_perm) {
+              int gate_half, const int* in_perm, const int* out_perm, int tc_passes) {
     B200_REQUIRE(w != nullptr && Cout > 0 && Cin > 0 && K > 0, "pack_conv: bad arguments");
     B200_REQUIRE(gate_half == 0 || 2 * gate_half == Cout, "pack_conv: gate_half must be Cout/2");
     std::vector<float> Wl((size_t)Cout * Cin * K), bl(Cout, 0.f);
@@ -515,10 +528,11 @@ int pack_conv(ConvLayer& L, const float* w, const float* bias, int Cout, int Cin
     L.dil = dil;
     L.pad = pad;
     L.ups = 1;
-    return pack_rows(L, Wl, bl, Cout, Cin, K);
+    return pack_rows(L, Wl, bl, Cout, Cin, K, tc_passes);
 }
 
-int pack_conv_transpose(ConvLayer& L, const float* w, const float* bias, int Cin, int Cout, int Kt, int s, int p) {
+int pack_conv_transpose(ConvLayer& L, const float* w, const float* bias, int Cin, int Cout, int Kt, int s, int p,
+                        int tc_passes) {
     // y[co, q*s+ph] = sum_ci sum_m x[ci, q-m] * w[ci, co, ph + p + m*s]   (0 <= ph+p+m*s < Kt)
     B200_REQUIRE(w != nullptr && s >= 1 && Kt >= 1, "pack_conv_transpose: bad arguments");
     auto floordiv = [](int a, int b) { return (a >= 0) ? a / b : -((-a + b - 1) / b); };
@@ -545,7 +559,7 @@ int pack_conv_transpose(ConvLayer& L, const float* w, const float* bias, int Cin
     L.ups = s;
     L.tr_kernel = Kt;
     L.tr_pad = p;
-    return pack_rows(L, Wl, bl, rows, Cin, K);
+    return pack_rows(L, Wl, bl, rows, Cin, K, tc_passes);
 }
 
 // ------------------------------------------------------------------ single-output-row conv (HiFiGAN conv_post)
@@ -743,8 +757,11 @@ static int try_launch_tc(const ConvLayer& L, const ConvIO& io, const ConvKArgs& 
         B200_CUDA_OK(cudaFuncSetAttribute(tc3::conv1d_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         B200_CUDA_OK(cudaFuncSetAttribute(tc3::conv1d_tc3s_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         B200_CUDA_OK(cudaFuncSetAttribute(tc3::conv1d_tc3x_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        B200_CUDA_OK(cudaFuncSetAttribute(tc3::conv1d_tc3_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        B200_CUDA_OK(cudaFuncSetAttribute(tc3::conv1d_tc3x_tf32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         for (int g : {2, 4})
-            B200_CUDA_OK(cudaFuncSetAttribute(tc3::grouped_kernel(g), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            for (bool x1 : {false, true})
+                B200_CUDA_OK(cudaFuncSetAttribute(tc3::grouped_kernel(g, x1), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
         int* flag = nullptr;
         B200_CUDA_OK(cudaHostAlloc((void**)&flag, sizeof(int), cudaHostAllocMapped | cudaHostAllocPortable));
         *flag = 0;
@@ -757,6 +774,9 @@ static int try_launch_tc(const ConvLayer& L, const ConvIO& io, const ConvKArgs& 
     B200_REQUIRE(*reinterpret_cast<volatile int*>(g_tc_err) == 0,
                  "tcgen05 conv: an earlier launch on device %d hit a pipeline timeout (its output is invalid)", dev);
     const int rows_pad = (tc::TT + (L.K - 1) * L.dil + 7) / 8 * 8;
+    // single-pass TF32 layers run the X1 twins of the same kernels.  Eligibility is always judged with the 3xTF32
+    // shared-memory size, so a layer takes the same family in either mode; the launch sizes what the kernel uses.
+    const bool x1 = L.tc_passes == 1;
     // ---- persistent kernel (needs 16-byte aligned activation rows for its cp.async staging; no input mask)
     const bool aligned = ((reinterpret_cast<uintptr_t>(a.x) & 15) == 0) && (a.x_cs % 4 == 0) && (a.x_bs % 4 == 0);
     const int n_rtiles = (L.Rows + L.tc_n - 1) / L.tc_n;
@@ -780,15 +800,15 @@ static int try_launch_tc(const ConvLayer& L, const ConvIO& io, const ConvKArgs& 
             t.rows_pad = rp; t.raw_w = rp + 4;
             t.B = io.B; t.n_ttiles = (a.Tq + t.tstep - 1) / t.tstep; t.n_rtiles = 1;
             t.err = g_tc_err;
-            size_t smemg = (tc3::smem_bytes3(rp, rp + 4) + 127) / 128 * 128;
+            size_t smemg = (tc3::smem_bytes3(rp, rp + 4, L.tc_passes) + 127) / 128 * 128;
             t.stage_off = (int)smemg;                          // partial-sum exchange tiles of the grouped epilogue
             smemg += tc3::GROUP_XCHG_BYTES;
             set_ragged(t, a, smemg);
             const long long tiles = (long long)t.B * t.n_ttiles;
             const int grid = (int)(tiles < num_sms ? tiles : num_sms);
-            B200_CUDA_OK(launch_tc3(tc3::grouped_kernel(G), grid, smemg, st, t));
+            B200_CUDA_OK(launch_tc3(tc3::grouped_kernel(G, x1), grid, smemg, st, t));
             count_launch();
-            dispatch_note(DISPATCH_TC3_GROUPED);
+            dispatch_note(x1 ? DISPATCH_TC3_GROUPED_TF32 : DISPATCH_TC3_GROUPED);
             B200_CUDA_OK(cudaGetLastError());
             return 0;
         }
@@ -815,11 +835,11 @@ static int try_launch_tc(const ConvLayer& L, const ConvIO& io, const ConvKArgs& 
         t.err = g_tc_err;
         static int staged = -1;
         if (staged < 0) { const char* e = getenv("B200TTS_STAGED"); staged = (e && atoi(e)) ? 1 : 0; }
-        size_t smem3 = tc3::smem_bytes3(rows_pad, rows_pad + 4);
+        size_t smem3 = tc3::smem_bytes3(rows_pad, rows_pad + 4, L.tc_passes);
         // staged (shared-memory transposed, coalesced) epilogue for K <= 3 layers.  It beat the r01 direct epilogue by 13 % on
         // those layers; since the direct epilogue prefetches without register copies (r02) the direct one wins
         // (decoder 17.2 -> 16.5 ms per bench step, same box A/B), so it is opt-in again: B200TTS_STAGED=1
-        if (staged && L.K <= 3 && L.ups == 1 && !t.gate && t.split == 0 && ((smem3 + 15) / 16 * 16 + tc3::STAGE_BYTES) <= 227 * 1024) {
+        if (staged && !x1 && L.K <= 3 && L.ups == 1 && !t.gate && t.split == 0 && ((smem3 + 15) / 16 * 16 + tc3::STAGE_BYTES) <= 227 * 1024) {
             t.stage = 1;
             t.stage_off = (int)((smem3 + 15) / 16 * 16);
             smem3 = (size_t)t.stage_off + tc3::STAGE_BYTES;
@@ -834,9 +854,11 @@ static int try_launch_tc(const ConvLayer& L, const ConvIO& io, const ConvKArgs& 
         set_ragged(t, a, smem3);
         const long long tiles = (long long)t.B * t.n_ttiles * t.n_rtiles;
         const int grid = (int)(tiles < num_sms ? tiles : num_sms);
-        B200_CUDA_OK(launch_tc3(t.stage ? tc3::conv1d_tc3s_kernel : plain_epi ? tc3::conv1d_tc3_kernel : tc3::conv1d_tc3x_kernel, grid, smem3, st, t));
+        tc3::Tc3Kernel k3 = t.stage ? tc3::conv1d_tc3s_kernel : plain_epi ? tc3::conv1d_tc3_kernel : tc3::conv1d_tc3x_kernel;
+        if (x1) k3 = plain_epi ? tc3::conv1d_tc3_tf32_kernel : tc3::conv1d_tc3x_tf32_kernel;
+        B200_CUDA_OK(launch_tc3(k3, grid, smem3, st, t));
         count_launch();
-        dispatch_note(t.stage ? DISPATCH_TC3_STAGED : DISPATCH_TC3);
+        dispatch_note(x1 ? DISPATCH_TC3_TF32 : t.stage ? DISPATCH_TC3_STAGED : DISPATCH_TC3);
         B200_CUDA_OK(cudaGetLastError());
         return 0;
     }

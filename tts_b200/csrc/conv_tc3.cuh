@@ -18,6 +18,11 @@
 //   warp  11         MMA       : converged warp, one elected lane issues 3 tcgen05.mma (lo*hi, hi*lo, hi*hi) per tap and
 //                                chunk and commits to mbarriers
 //
+// Single-pass TF32 mode (template flag X1, the opt-in `tf32` precision of the HiFiGAN decoder): the producers round the
+// activation to TF32 (cvt.rna: nearest, ties away from zero) instead of splitting it, the packer rounds the weights with
+// the same rule, there are no lo slabs (half the activation stage, 4 KB tap blocks) and one MMA per tap.  Everything
+// else -- schedule, barriers, partial-tile N, epilogues -- is the same code.
+//
 // Grouped mode (GRP = 2 / 4) for narrow layers (exactly 64 / 32 output rows, the last two HiFiGAN stages): the 128
 // MMA rows are GRP tap-groups x (128/GRP) channels -- row g * (128/GRP) + c carries the weights of channel c for taps
 // g, g+GRP, g+2*GRP, ... so one instruction stream of ceil(K/GRP) "tap blocks" (B shifted by GRP*dil rows per block)
@@ -54,7 +59,7 @@ constexpr int RAWS = 324;         // raw (cp.async) row stride in floats: the wi
 #endif
 constexpr int NRAW = TC3_NRAW;    // raw (cp.async) ring depth
 constexpr int NA2 = TC3_NA2;      // transformed activation stages
-constexpr int NB2 = TC3_NB2;      // weight ring depth (one 8 KB tap block per slot)
+constexpr int NB2 = TC3_NB2;      // weight ring depth (one tap block per slot: 8 KB, 4 KB single-pass)
 #ifndef TC3_RDEPTH
 #define TC3_RDEPTH 2
 #endif
@@ -70,7 +75,7 @@ constexpr int NTHREADS2 = 32 * (W_EPI2 + 4);
 struct Tc3Args {
     const float* x; long long x_bs; int x_cs; int Tin;
     float in_slope;
-    const float* w;            // packed [row_tile][chunk][tap]{hi[2][128][4], lo[2][128][4]}
+    const float* w;            // packed [row_tile][chunk][tap]{hi[2][128][4], lo[2][128][4]} (single pass: {w[2][128][4]})
     const float* bias;
     const float* cond; long long cond_bs;
     int Cin, K, dil, pad, Rows, N;
@@ -105,9 +110,11 @@ struct Tc3Args {
     int pref_off;               // byte offset in dynamic shared memory of the (B + 1)-entry tile prefix table
 };
 
-static inline size_t smem_bytes3(int rows_pad, int raw_w) {
+// passes: 3 (3xTF32, {hi,lo} slabs) or 1 (single-pass TF32, one slab pair per activation stage and weight block)
+static inline size_t smem_bytes3(int rows_pad, int raw_w, int passes = 3) {
     (void)raw_w;     // raw rows are stored at the fixed stride RAWS
-    return (size_t)NRAW * KC2 * RAWS * 4 + (size_t)NA2 * (4 * rows_pad * 16) + (size_t)NB2 * (4 * MROWS * 16) + 512;
+    const size_t slabs = passes == 1 ? 2 : 4;
+    return (size_t)NRAW * KC2 * RAWS * 4 + (size_t)NA2 * (slabs * rows_pad * 16) + (size_t)NB2 * (slabs * MROWS * 16) + 512;
 }
 static inline size_t ragged_table_bytes(int B) { return ((size_t)(B + 1) * sizeof(int) + 15) / 16 * 16; }
 
@@ -141,6 +148,12 @@ __device__ __forceinline__ void tmem_ld_nowait(uint32_t taddr, uint32_t* r) {   
 __device__ __forceinline__ void tmem_st16_zero(uint32_t taddr) {
     const uint32_t z = 0u;
     asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1,%1};" ::"r"(taddr), "r"(z) : "memory");
+}
+// round to TF32, nearest with ties away from zero (the packer's host rounding, conv1d.cu tf32_rna, is the same rule)
+__device__ __forceinline__ float tf32_rna(float x) {
+    uint32_t r;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+    return __uint_as_float(r);
 }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
@@ -498,16 +511,18 @@ __device__ __noinline__ void general_tile_call(const Tc3Args& a_ref, unsigned ch
     general_tile_body<STAGED>(a, smem, tmem_base, acc_cols, b, rt, q0, buf, lq, half, lane, warp);
 }
 
-template <int GRP, bool STAGED = false, bool LEAN = true>   // GRP: tap groups stacked in the 128 MMA rows (1 = plain); STAGED: wide-layer
+template <int GRP, bool STAGED = false, bool LEAN = true, bool X1 = false>   // GRP: tap groups stacked in the 128 MMA rows (1 = plain); STAGED: wide-layer
                                           // epilogue through per-warp shared tiles; LEAN: plain-layer kernel (lean epilogue inline, general
-                                          // one out of line) -- false for the WaveNet / masked / transposed layers (general epilogue inline)
+                                          // one out of line) -- false for the WaveNet / masked / transposed layers (general epilogue inline);
+                                          // X1: single-pass TF32 (one rounded slab pair per operand, one MMA per tap)
 __device__ __forceinline__ void tc3_body(const Tc3Args& a) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int ROWS = a.rows_pad, RAWW = a.raw_w, K = a.KJ;
     const uint32_t rawStage = (uint32_t)KC2 * RAWS * 4;
-    const uint32_t slabA = (uint32_t)ROWS * 16, stageA = 4 * slabA;     // hi[2] + lo[2]
-    const uint32_t slabB = (uint32_t)MROWS * 16, stageB = 4 * slabB;   // one tap block: {hi,lo}[2 slabs][128 rows][16 B]
+    constexpr uint32_t NSL = X1 ? 2 : 4;                                 // slabs per stage / tap block
+    const uint32_t slabA = (uint32_t)ROWS * 16, stageA = NSL * slabA;   // hi[2] + lo[2]  (single pass: x[2])
+    const uint32_t slabB = (uint32_t)MROWS * 16, stageB = NSL * slabB;  // one tap block: {hi,lo}[2 slabs][128 rows][16 B]
     unsigned char* smRaw = smem;
     unsigned char* smA = smRaw + NRAW * rawStage;
     unsigned char* smB = smA + NA2 * stageA;
@@ -713,6 +728,14 @@ __device__ __forceinline__ void tc3_body(const Tc3Args& a) {
 #pragma unroll
                 for (int e = 0; e < MAXI; ++e) {           // ... then prologue, hi/lo split and the two 16-byte stores
                     if (i_raw[e] < 0) continue;
+                    if constexpr (X1) {                     // single pass: leaky ReLU, round to TF32, one store
+                        float4 v;
+                        float* pv = &v.x;
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) pv[i] = tf32_rna(fmaxf(u[e][i], u[e][i] * slope));
+                        *reinterpret_cast<float4*>(base + i_dst[e]) = v;
+                        continue;
+                    }
                     float4 hi, lo;
                     float* ph = &hi.x; float* pl = &lo.x;
 #pragma unroll
@@ -846,9 +869,13 @@ __device__ __forceinline__ void tc3_body(const Tc3Args& a) {
                         const uint64_t w_hi = wdesc, w_lo = wdesc + wlo_off;
                         if (leader) {
                             if (!no_mma) {
-                                mma_tf32(dcol, w_hi, xl, idesc_t, acc);                   // small terms first
-                                mma_tf32(dcol, w_lo, xh, idesc_t, 1u);
-                                mma_tf32(dcol, w_hi, xh, idesc_t, 1u);
+                                if constexpr (X1) {
+                                    mma_tf32(dcol, w_hi, xh, idesc_t, acc);
+                                } else {
+                                    mma_tf32(dcol, w_hi, xl, idesc_t, acc);               // small terms first
+                                    mma_tf32(dcol, w_lo, xh, idesc_t, 1u);
+                                    mma_tf32(dcol, w_hi, xh, idesc_t, 1u);
+                                }
                             }
                             if (thread_arrive) mbar_arrive(bempty); else mma_commit(bempty);
                         }
@@ -1091,10 +1118,18 @@ __global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3s_kernel(const __grid_
 __global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3x_kernel(const __grid_constant__ Tc3Args a) { tc3_body<1, false, false>(a); }   // gate / split / mask / polyphase
 template <int GRP>
 __global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3g_kernel(const __grid_constant__ Tc3Args a) { tc3_body<GRP>(a); }
+// single-pass TF32 twins (no staged one: a single-pass layer never takes the staged epilogue)
+__global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3_tf32_kernel(const __grid_constant__ Tc3Args a) { tc3_body<1, false, true, true>(a); }
+__global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3x_tf32_kernel(const __grid_constant__ Tc3Args a) { tc3_body<1, false, false, true>(a); }
+template <int GRP>
+__global__ void __launch_bounds__(NTHREADS2, 1) conv1d_tc3g_tf32_kernel(const __grid_constant__ Tc3Args a) { tc3_body<GRP, false, true, true>(a); }
 
 typedef void (*Tc3Kernel)(const Tc3Args);
-// grouped kernel for 2 / 4 tap groups (any dilation with (GRP - 1) * dil <= 15)
-static inline Tc3Kernel grouped_kernel(int grp) { return grp == 2 ? conv1d_tc3g_kernel<2> : conv1d_tc3g_kernel<4>; }
+// grouped kernel for 2 / 4 tap groups (any dilation with (GRP - 1) * dil <= 15); x1: single-pass TF32
+static inline Tc3Kernel grouped_kernel(int grp, bool x1 = false) {
+    if (x1) return grp == 2 ? conv1d_tc3g_tf32_kernel<2> : conv1d_tc3g_tf32_kernel<4>;
+    return grp == 2 ? conv1d_tc3g_kernel<2> : conv1d_tc3g_kernel<4>;
+}
 constexpr int GROUP_XCHG_BYTES = 2 * 2 * 128 * 16 * 4;   // grouped epilogue: per column half two buffers of [128 rows][16] floats
 
 }  // namespace tc3

@@ -14,8 +14,9 @@ struct Hifigan {
     ConvLayer conv_pre, cond, conv_post;
     std::vector<ConvLayer> ups;
     std::vector<std::vector<ConvLayer>> rb_c1, rb_c2;
+    int precision = B200TTS_PRECISION_FP32;   // B200TTS_PRECISION_*: how the tensor-core layers were packed
     ~Hifigan();
-    int init(const b200tts_hifigan_config& cfg, const float* const* w, int nw);
+    int init(const b200tts_hifigan_config& cfg, const float* const* w, int nw, int precision = B200TTS_PRECISION_FP32);
     void stage_dims(int T, std::vector<int>& C, std::vector<int>& L) const;
     size_t workspace_bytes(int B, int T) const;
     int out_len(int T) const;

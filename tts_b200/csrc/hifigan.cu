@@ -15,8 +15,13 @@ Hifigan::~Hifigan() {
 }
 
 // weights: host pointers, canonical order (see include/tts_b200.h)
-int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int nw) {
+int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int nw, int prec) {
     c = cfg;
+    B200_REQUIRE(prec == B200TTS_PRECISION_FP32 || prec == B200TTS_PRECISION_TF32, "hifigan: unknown precision %d", prec);
+    precision = prec;
+    // conv_pre, the upsamplers and the ResBlock convs are the tensor-core layers: packed for one pass in TF32 mode.
+    // cond_layer and conv_post run on the FP32 kernels in either mode.
+    const int tp = prec == B200TTS_PRECISION_TF32 ? 1 : 3;
     B200_REQUIRE(c.num_upsamples >= 1 && c.num_upsamples <= 8 && c.num_kernels >= 1 && c.num_kernels <= 8 &&
                      c.num_dilations >= 1 && c.num_dilations <= 8,
                  "hifigan: unsupported config");
@@ -25,7 +30,7 @@ int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int 
                        c.num_upsamples * c.num_kernels * c.num_dilations * (type1 ? 4 : 2) + 2;
     B200_REQUIRE(nw == expect, "hifigan: expected %d weight tensors, got %d", expect, nw);
     int i = 0;
-    int rc = pack_conv(conv_pre, w[i], w[i + 1], c.upsample_initial_channel, c.in_channels, 7, 1, 3);
+    int rc = pack_conv(conv_pre, w[i], w[i + 1], c.upsample_initial_channel, c.in_channels, 7, 1, 3, 0, nullptr, nullptr, tp);
     if (rc) return rc;
     i += 2;
     if (c.cond_channels > 0) {
@@ -39,7 +44,7 @@ int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int 
     int ch = c.upsample_initial_channel;
     for (int s = 0; s < c.num_upsamples; ++s) {
         const int u = c.upsample_factors[s], k = c.upsample_kernel_sizes[s];
-        rc = pack_conv_transpose(ups[s], w[i], w[i + 1], ch, ch / 2, k, u, (k - u) / 2);
+        rc = pack_conv_transpose(ups[s], w[i], w[i + 1], ch, ch / 2, k, u, (k - u) / 2, tp);
         if (rc) return rc;
         i += 2;
         ch /= 2;
@@ -51,11 +56,11 @@ int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int 
             if (type1) v2.resize(c.num_dilations);
             for (int n = 0; n < c.num_dilations; ++n) {
                 const int d = c.resblock_dilations[j][n];
-                rc = pack_conv(v1[n], w[i], w[i + 1], ch, ch, rk, d, (rk * d - d) / 2);
+                rc = pack_conv(v1[n], w[i], w[i + 1], ch, ch, rk, d, (rk * d - d) / 2, 0, nullptr, nullptr, tp);
                 if (rc) return rc;
                 i += 2;
                 if (type1) {
-                    rc = pack_conv(v2[n], w[i], w[i + 1], ch, ch, rk, 1, (rk - 1) / 2);
+                    rc = pack_conv(v2[n], w[i], w[i + 1], ch, ch, rk, 1, (rk - 1) / 2, 0, nullptr, nullptr, tp);
                     if (rc) return rc;
                     i += 2;
                 }
@@ -63,7 +68,7 @@ int Hifigan::init(const b200tts_hifigan_config& cfg, const float* const* w, int 
         }
     }
     rc = pack_conv(conv_post, w[i], w[i + 1], c.out_channels, ch, 7, 1, 3);
-    // the MRF / pre convs carry ~97% of the FLOPs: run them on the tcgen05 3xTF32 kernel
+    // the MRF / pre convs carry ~97% of the FLOPs: run them on the tcgen05 kernels (3xTF32, or single pass in TF32 mode)
     conv_pre.allow_tc = true;
     for (auto& l : ups) l.allow_tc = true;
     for (auto& v : rb_c1) for (auto& l : v) l.allow_tc = true;

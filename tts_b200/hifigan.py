@@ -5,6 +5,11 @@ Same constructor signature, same ``state_dict`` keys (the torch modules below ar
 containers -- weight-norm parametrizations included -- so reference checkpoints load unchanged),
 same ``forward(x, g=None)`` / ``inference(c)`` / ``remove_weight_norm()`` / ``load_checkpoint``.
 The arithmetic runs in libtts_b200.so (b200tts_hifigan_forward); there is no PyTorch fallback.
+
+``precision`` selects the numerics of the tensor-core convolutions (conv_pre, upsamplers, ResBlocks): ``"fp32"``
+(default, 3xTF32: waveform within 1e-4 RMS of an fp32 computation) or ``"tf32"`` (single-pass TF32 with operands
+rounded to nearest -- what the reference gets from cuDNN with torch's default ``allow_tf32`` -- and faster).  It is a
+plain attribute, not part of ``state_dict``; torch's global TF32 flags are deliberately not consulted.
 """
 import ctypes
 
@@ -100,10 +105,23 @@ class HifiganGenerator(nn.Module):
             remove_parametrizations(self.conv_post, "weight")
         self._handle = None
         self._handle_device = None
+        self._precision = "fp32"
         # a parent's load_state_dict never calls a child's load_state_dict() override (it recurses through
         # _load_from_state_dict), so the packed handle is dropped from a pre-hook: Vits.load_checkpoint twice in a row
         # must not keep the first checkpoint's decoder weights
         self._register_load_state_dict_pre_hook(lambda *a, **k: self._drop_handle())
+
+    # ------------------------------------------------------------------ numerics
+    @property
+    def precision(self):
+        """``"fp32"`` (3xTF32, default) or ``"tf32"`` (single-pass TF32) for the tensor-core layers."""
+        return self._precision
+
+    @precision.setter
+    def precision(self, value):
+        _lib.precision_id(value)              # validates (ValueError) without loading the CUDA library
+        self._drop_handle()                   # the packed handle holds the weights in the old mode's format
+        self._precision = value
 
     # ------------------------------------------------------------------ engine handle
     def _drop_handle(self):
@@ -168,7 +186,8 @@ class HifiganGenerator(nn.Module):
         arr = (ctypes.c_void_p * len(tensors))(*[None if t is None else t.data_ptr() for t in tensors])
         handle = ctypes.c_void_p()
         with torch.cuda.device(device):
-            rc = _lib.lib().b200tts_hifigan_create(ctypes.byref(cfg), arr, len(tensors), ctypes.byref(handle))
+            rc = _lib.lib().b200tts_hifigan_create_ex(ctypes.byref(cfg), arr, len(tensors),
+                                                      _lib.precision_id(self._precision), ctypes.byref(handle))
         _lib.check(rc, "hifigan_create")
         self._handle, self._handle_device = handle, device
         return handle
